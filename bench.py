@@ -79,6 +79,19 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+def dump_outputs(path: str, arrays: dict, limit: int) -> None:
+    """Writes each tensor as float32 `path`/<name>.npy.  A tensor larger than its share of `limit` bytes is replaced by a
+    fixed seeded sample of its flattened elements, so that runs with the same arguments stay comparable."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    n_max = (limit - 4096 * len(arrays)) // 4 // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() > n_max:
+            a = a.reshape(-1)[torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:n_max].sort().values]
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+
+
 def plan_shard(rank: int, world: int, n_frames: int):
     from hallo_b200.dist import plan_shard as ps
     return ps(rank, world, n_frames)
@@ -320,7 +333,13 @@ def main():
     ap.add_argument("--emulate-shard", type=int, default=0, metavar="R",
                     help="single GPU: run the workload of ONE rank of an R-rank job (cond half, first frame group, no "
                          "collectives) -- for ncu / op profiles of the sharded shapes; the JSON line is marked invalid")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write the latents the last timed step returned (float32, [1, 4, frames, "
+                         "size, size]) to DIR/latents.npy, or each rank's frames to DIR/latents_rank<r>.npy; weights and "
+                         "inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.windows > 0 or args.profiler_range):
+        ap.error("--dump-outputs writes the outputs of the timed denoising steps of the GPU run")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -483,6 +502,8 @@ def main():
     barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"latents" if world == 1 else f"latents_rank{rank}": eng.latents}, (64 << 20) // world)
     ms_step = ms_total / K
     fps = args.frames / (N_DDIM * ms_step * 1e-3)
 

@@ -7,6 +7,8 @@ Fixtures (small, committed):
   unet_fwd_h{H}_f{F}.pt           reference UNet3D forward output on hallo_b200.synth inputs/weights
                                   (fp32, shipped branch, read-mode reader with synthetic fp16 banks)
                                   + per-block output statistics + input checksums
+  refnet_h16_f32.pt               reference UNet2D + write-mode control at latent 16x16, fp32 (see make_refnet_h16)
+  process_audio_emb.pt            scripts/inference.py process_audio_emb on a seeded embedding
 The weights/inputs are NOT stored: they are regenerated from seeds by hallo_b200/synth.py; the stored
 checksums detect generator drift.
 """
@@ -32,7 +34,9 @@ CASES = [dict(h=8, f=2, seed=42, t=999, ms=(1.0, 0.9, 1.1)),
          # level sizes (L = 9216, 2304, 576, 144); run with `--only h64_f2 h64_f16 h96_f2` (f=16 takes ~3 min on 8 cores)
          dict(h=64, f=2, seed=45, t=777, ms=(1.0, 0.7, 1.3)),
          dict(h=64, f=16, seed=46, t=499, ms=(1.1, 0.9, 1.0)),
-         dict(h=96, f=2, seed=47, t=261, ms=(0.9, 1.1, 1.0))]
+         dict(h=96, f=2, seed=47, t=261, ms=(0.9, 1.1, 1.0)),
+         # fp32 cross-check of the port against the reference at a third timestep and uneven motion scales
+         dict(h=8, f=3, seed=7, t=123, ms=(0.7, 1.3, 1.0))]
 
 
 def checksum(t: torch.Tensor) -> float:
@@ -67,6 +71,44 @@ def make_refnet():
     print("wrote", path, tuple(out.shape), "std", float(out.std()))
 
 
+def make_refnet_h16():
+    """refnet_h16_f32.pt: the same reference ReferenceNet at latent 16x16 (seed 11), kept in fp32 so that the port can be
+    held to 2e-5: the bank pairing order, the absolute sums of the output and of every bank, and fixed seeded samples
+    (flat indices stored next to the values) of 16384 output elements and 2048 elements per bank; the full tensors
+    take 19 MB."""
+    cfg = UNetConfig()
+    unet = ref_host.build_reference_unet2d()
+    unet.load_state_dict(synth_state_dict_2d(cfg), strict=True)
+    c = dict(h=16, seed=11)
+    inp = synth_refnet_inputs(cfg, c["h"], c["h"], seed=c["seed"])
+    out, banks, names = ref_host.run_reference_net(unet, inp)
+    g = torch.Generator().manual_seed(0)
+
+    def sample(t, n):
+        i = torch.randperm(t.numel(), generator=g)[:n].sort().values
+        return dict(index=i.int(), values=t.float().reshape(-1)[i], abs_sum=checksum(t))
+    fx = dict(case=c, out=sample(out, 16384), bank_order=names, banks={n: sample(b, 2048) for n, b in zip(names, banks)},
+              input_checksums=dict(sample=checksum(inp["sample"])), torch_version=torch.__version__)
+    path = os.path.join(GOLD, "refnet_h16_f32.pt")
+    torch.save(fx, path)
+    print("wrote", path, tuple(out.shape))
+
+
+def make_process_audio_emb():
+    """process_audio_emb.pt: process_audio_emb of the reference's scripts/inference.py (the function alone, executed
+    without importing the script's dependencies) on a seeded (37, 12, 8) embedding."""
+    import ast
+    src = open(os.path.join(ref_host.REFERENCE_ROOT, "scripts", "inference.py")).read()
+    fn = next(n for n in ast.parse(src).body if isinstance(n, ast.FunctionDef) and n.name == "process_audio_emb")
+    ns = {"torch": torch}
+    exec(compile(ast.Module(body=[fn], type_ignores=[]), "inference.py", "exec"), ns)
+    emb = torch.randn(37, 12, 8, generator=torch.Generator().manual_seed(0))
+    fx = dict(case=dict(shape=(37, 12, 8), seed=0), input_checksum=checksum(emb), out=ns["process_audio_emb"](emb))
+    path = os.path.join(GOLD, "process_audio_emb.pt")
+    torch.save(fx, path)
+    print("wrote", path, tuple(fx["out"].shape))
+
+
 def make_audio_proj():
     """audio_proj_f4.pt: the UNMODIFIED reference AudioProjModel (hallo/models/audio_proj.py) on synth weights, 4 frames."""
     from hallo_b200.synth import synth_audio_proj_state_dict
@@ -87,21 +129,16 @@ def make_audio_proj():
 
 def main():
     only = sys.argv[sys.argv.index("--only") + 1:] if "--only" in sys.argv else None
-    if only is not None and "audio_proj" in only:
-        torch.set_num_threads(host_threads())
-        make_audio_proj()
-        only = [o for o in only if o != "audio_proj"]
-        if not only:
-            return
-    if only is not None and "refnet" in only:
-        torch.set_num_threads(host_threads())
-        os.makedirs(GOLD, exist_ok=True)
-        make_refnet()
-        only = [o for o in only if o != "refnet"]
-        if not only:
-            return
     torch.set_num_threads(host_threads())
     os.makedirs(GOLD, exist_ok=True)
+    others = {"refnet": make_refnet, "refnet_h16": make_refnet_h16, "audio_proj": make_audio_proj,
+              "process_audio_emb": make_process_audio_emb}
+    if only is not None:
+        for name in [o for o in only if o in others]:
+            others[name]()
+        only = [o for o in only if o not in others]
+        if not only:
+            return
     cfg = UNetConfig()
     unet = ref_host.build_reference_unet()
     keys = {k: list(v.shape) for k, v in unet.state_dict().items()}
@@ -140,8 +177,8 @@ def main():
         torch.save(fx, path)
         print("wrote", path, tuple(out.shape), "std", float(out.std()))
     if only is None:
-        make_refnet()
-        make_audio_proj()
+        for make in others.values():
+            make()
 
 
 if __name__ == "__main__":
