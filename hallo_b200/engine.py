@@ -10,6 +10,9 @@ matrices, with all weights pre-packed once and all step-invariant work hoisted o
                    inputs, masks, mask_cond_fea, motion_scale-folded zero-conv weights
   per step       : the kernels in `_forward()` -- captured once into a CUDA graph and replayed.
 
+`_forward()` is `_walk()` (time embedding, conv_in, down / mid / up blocks) plus the conv_out head.  The ReferenceNet
+(refnet.py) runs the same `_walk()`: its block list has no audio / motion modules and its window no reference K/V.
+
 Layout: every activation is a token matrix [rows, C]; rows are ordered (cfg_half, frame, pixel) --
 i.e. the reference's `(b f) (h w) c` -- so NCHW<->NLC permutes, `rearrange`s and `torch.cat`s of the
 reference disappear (channel concats become two-source reads, frame concats become row offsets).
@@ -27,7 +30,7 @@ from __future__ import annotations
 import math
 from dataclasses import dataclass
 import os
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, Optional, Sequence, Tuple
 
 import torch
 
@@ -51,14 +54,14 @@ class Shard:
 
 class PackedWeights:
     """Device-resident, kernel-ready copies of the state dict (packed once per model load)."""
-    kind = "3d"        # refnet.ReferenceNetWeights sets "2d": resnets + spatial blocks only, no output head
+    build_blocks = staticmethod(build_blocks)     # the layers to pack and run; refnet.ReferenceNetWeights: the UNet2D's
 
     def __init__(self, sd: Dict[str, torch.Tensor], cfg: UNetConfig, device, dtype):
         self.cfg = cfg
         self.dtype = dtype
         self.device = device
         self.t: Dict[str, torch.Tensor] = {}
-        blocks = build_blocks(cfg)
+        blocks = self.build_blocks(cfg)
         self.blocks = blocks
 
         def dev(x):
@@ -80,14 +83,21 @@ class PackedWeights:
             put(f"{name}.w", ops.pack_conv3x3_weight(sd[f"{name}.weight"]))
             put(f"{name}.b", sd[f"{name}.bias"])
 
-        def qkv(name, out_name):
-            put(out_name, torch.cat([sd[f"{name}.to_q.weight"], sd[f"{name}.to_k.weight"], sd[f"{name}.to_v.weight"]], 0))
-
-        def ff(name):
-            wi, bi = ops.pack_geglu_weight(sd[f"{name}.net.0.proj.weight"], sd[f"{name}.net.0.proj.bias"])
-            put(f"{name}.w1", wi)
-            put(f"{name}.b1", bi)
-            lin(f"{name}.net.2")
+        def transformer(name, norms, self_attns):
+            """The part the spatial, audio and motion transformers share: GroupNorm, proj_in / proj_out, the block's
+            LayerNorms, each self-attention's fused QKV and to_out, the GEGLU feed-forward."""
+            tb = f"{name}.transformer_blocks.0"
+            norm(f"{name}.norm"); lin(f"{name}.proj_in"); lin(f"{name}.proj_out")
+            for k in norms:
+                norm(f"{tb}.{k}")
+            for a in self_attns:
+                put(f"{tb}.{a}.qkv", torch.cat([sd[f"{tb}.{a}.to_{p}.weight"] for p in "qkv"], 0))
+                lin(f"{tb}.{a}.to_out.0")
+            wi, bi = ops.pack_geglu_weight(sd[f"{tb}.ff.net.0.proj.weight"], sd[f"{tb}.ff.net.0.proj.bias"])
+            put(f"{tb}.ff.w1", wi)
+            put(f"{tb}.ff.b1", bi)
+            lin(f"{tb}.ff.net.2")
+            return tb
 
         # stem / head
         w_in = sd["conv_in.weight"]                                  # [C0, Cl, 3, 3] -> [C0, 64], k = tap*Cl + c
@@ -101,7 +111,7 @@ class PackedWeights:
         put("conv_in.b", sd["conv_in.bias"])
         lin("time_embedding.linear_1")
         lin("time_embedding.linear_2")
-        if self.kind == "3d":
+        if "conv_out.weight" in sd:                                    # the UNet2D ends at the last up block
             norm("conv_norm_out")
             w_out = ops.pack_conv3x3_weight(sd["conv_out.weight"])       # [Cl, 9*C0] -> padded to 8 rows
             wo = torch.zeros(8, w_out.shape[1], dtype=w_out.dtype, device=w_out.device)
@@ -134,26 +144,13 @@ class PackedWeights:
             for l in b.layers:
                 resnet(l.resnet)
                 if l.attn:
-                    n = l.attn
-                    tb = f"{n}.transformer_blocks.0"
-                    norm(f"{n}.norm"); lin(f"{n}.proj_in"); lin(f"{n}.proj_out")
-                    for k in ("norm1", "norm2", "norm3"):
-                        norm(f"{tb}.{k}")
-                    qkv(f"{tb}.attn1", f"{tb}.attn1.qkv")
+                    tb = transformer(l.attn, ("norm1", "norm2", "norm3"), ("attn1",))
                     put(f"{tb}.attn1.kv", torch.cat([sd[f"{tb}.attn1.to_k.weight"], sd[f"{tb}.attn1.to_v.weight"]], 0))
-                    lin(f"{tb}.attn1.to_out.0")
                     put(f"{tb}.attn2.q", sd[f"{tb}.attn2.to_q.weight"])
                     put(f"{tb}.attn2.kv", torch.cat([sd[f"{tb}.attn2.to_k.weight"], sd[f"{tb}.attn2.to_v.weight"]], 0))
                     lin(f"{tb}.attn2.to_out.0")
-                    ff(f"{tb}.ff")
-                if l.audio and self.kind == "3d":
-                    n = l.audio
-                    tb = f"{n}.transformer_blocks.0"
-                    norm(f"{n}.norm"); lin(f"{n}.proj_in"); lin(f"{n}.proj_out")
-                    for k in ("norm1", "norm2", "norm3"):
-                        norm(f"{tb}.{k}")
-                    qkv(f"{tb}.attn1", f"{tb}.attn1.qkv")
-                    lin(f"{tb}.attn1.to_out.0")
+                if l.audio:
+                    tb = transformer(l.audio, ("norm1", "norm2", "norm3"), ("attn1",))
                     put(f"{tb}.attn2.q3", torch.cat([sd[f"{tb}.attn2_{r}.to_q.weight"] for r in range(3)], 0))
                     put(f"{tb}.attn2.kv6", torch.cat([torch.cat([sd[f"{tb}.attn2_{r}.to_k.weight"],
                                                                  sd[f"{tb}.attn2_{r}.to_v.weight"]], 0)
@@ -166,19 +163,12 @@ class PackedWeights:
                          for r in ("full", "face", "lip")], 0).to(device)
                     self.t[f"{tb}.zero.b"] = torch.stack([sd[f"{tb}.zero_conv_{r}.bias"].float()
                                                           for r in ("full", "face", "lip")], 0).to(device)
-                    ff(f"{tb}.ff")
-                if l.motion and l.motion_executed and self.kind == "3d":
-                    tt = f"{l.motion}.temporal_transformer"
-                    tb = f"{tt}.transformer_blocks.0"
-                    norm(f"{tt}.norm"); lin(f"{tt}.proj_in"); lin(f"{tt}.proj_out")
+                if l.motion_executed:
+                    tb = transformer(f"{l.motion}.temporal_transformer", ("norms.0", "norms.1", "ff_norm"),
+                                     ("attention_blocks.0", "attention_blocks.1"))
                     for a in range(2):
-                        norm(f"{tb}.norms.{a}")
-                        qkv(f"{tb}.attention_blocks.{a}", f"{tb}.attention_blocks.{a}.qkv")
-                        lin(f"{tb}.attention_blocks.{a}.to_out.0")
                         self.t[f"{tb}.attention_blocks.{a}.pe"] = \
                             sd[f"{tb}.attention_blocks.{a}.pos_encoder.pe"][0].float().to(device).contiguous()
-                    norm(f"{tb}.ff_norm")
-                    ff(f"{tb}.ff")
             if b.downsampler:
                 conv3(f"{b.downsampler}.conv")
             if b.upsampler:
@@ -360,6 +350,7 @@ class DenoiseEngine:
         aud2 = aud.reshape(nb * fl * aud.shape[2], aud.shape[3]).contiguous()
         ehs2 = ehs.reshape(nb * ehs.shape[1], ehs.shape[2]).contiguous()
         win["n_img_tokens"] = ehs.shape[1]
+        win["kvimg_frame_div"] = fl                    # the local rows of CFG half b read image K/V rows of batch b
         win["n_aud_tokens"] = aud.shape[2]
         mcf = mask_cond_fea.to(dev, dt)[halves][:, :, fr_idx]                 # [nb, C0, fl, h, w]
         self._wset("mask_cond", mcf.permute(0, 2, 3, 4, 1).reshape(-1, mcf.shape[1]).contiguous())
@@ -486,7 +477,13 @@ class DenoiseEngine:
         ops.gemm(g, W[f"{name}.net.2.w"], out, bias=W[f"{name}.net.2.b"], residual=x)
         return out
 
+    def _norm1_tag(self, name: str) -> str:
+        """Buffer of the spatial transformer's norm1 output (the ReferenceNet banks it)."""
+        return "ln"
+
     def _spatial(self, name: str, x, level: int, C: int, out_tag: str):
+        """Transformer3DModel + BasicTransformerBlock: self-attention (+ the window's reference K/V where it has them),
+        image cross-attention on the window's image K/V, GEGLU feed-forward."""
         W, B, win, H = self.W, self.B, self.window, self.cfg.heads
         L = self.L(level)
         M = B * L
@@ -495,13 +492,13 @@ class DenoiseEngine:
         self._gn(x, f"{name}.norm", t, B, L, 1e-6, False)
         h = self.buf("tf.h0", M, C)
         ops.gemm(t, W[f"{name}.proj_in.w"], h, bias=W[f"{name}.proj_in.b"])
-        n1 = self._ln(h, f"{tb}.norm1", "ln")
+        n1 = self._ln(h, f"{tb}.norm1", self._norm1_tag(name))
         qkv = self.buf("tf.qkv", M, 3 * C)
         ops.gemm(n1, W[f"{tb}.attn1.qkv"], qkv)
         a = self.buf("tf.attn", M, C)
-        kvref = win[f"{name}.kvref"]
-        ops.attention(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], a, heads=H, L=L, kref=kvref[:, :C], vref=kvref[:, C:],
-                      ref_index=win["ref_index"])
+        kvref = win.get(f"{name}.kvref")
+        ref = {} if kvref is None else dict(kref=kvref[:, :C], vref=kvref[:, C:], ref_index=win["ref_index"])
+        ops.attention(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], a, heads=H, L=L, **ref)
         h1 = self.buf("tf.h1", M, C)
         ops.gemm(a, W[f"{tb}.attn1.to_out.0.w"], h1, bias=W[f"{tb}.attn1.to_out.0.b"], residual=h)
         n2 = self._ln(h1, f"{tb}.norm2", "ln")
@@ -510,7 +507,7 @@ class DenoiseEngine:
         kvi = win[f"{name}.kvimg"]
         a2 = self.buf("tf.attn", M, C)
         ops.cross_attention(q2, kvi[:, :C], kvi[:, C:], a2, frames=B, tokens=L, heads=H, head_dim=C // H,
-                            n_keys=win["n_img_tokens"], kv_frame_div=self.fl)
+                            n_keys=win["n_img_tokens"], kv_frame_div=win["kvimg_frame_div"])
         h2 = self.buf("tf.h2", M, C)
         ops.gemm(a2, W[f"{tb}.attn2.to_out.0.w"], h2, bias=W[f"{tb}.attn2.to_out.0.b"], residual=h1)
         h3 = self._ff(h2, f"{tb}.ff", f"{tb}.norm3", "tf.h3")
@@ -560,59 +557,32 @@ class DenoiseEngine:
 
           in : GroupNorm of the local frames; its apply pass stores each row into the pixel owner's x18 over NVLink
                (ops.groupnorm_scatter) -> flag barrier
-          mid: proj_in, 2 x {LN + PE, QKV, temporal attention over the nm + f frames, to_out}, FF -- all rank-local,
-               no replicated motion-frame rows
+          mid: `_motion_body` over the nm + f frames of Lg pixels -- all rank-local, no replicated motion-frame rows
           out: proj_out GEMM whose epilogue stores every (frame, pixel) row into the frame owner's `recv`
                (hb_row_scatter) -> flag barrier -> out = recv + x (the module's residual)
 
         exchange == "nccl" performs the same two swaps with all_to_all_single (A/B baseline); emulate_group fills the
         peers' rows with copies of the local ones (single-GPU profile of one rank's shapes)."""
-        W, win, H, sh = self.W, self.window, self.cfg.heads, self.shard
+        W = self.W
         nb, nm, fl, f, R, me = self.nb, self.nm, self.fl, self.f, self.R, self.me
         L = self.L(level)
         Lg, F18 = L // R, nm + f
-        M18 = nb * F18 * Lg
         tt = f"{name}.temporal_transformer"
-        tb = f"{tt}.transformer_blocks.0"
-        x18 = self._x18(name, M18, C)
-        ws = self._gn_ws()
-        esz = x.element_size()
+        x18 = self._x18(name, nb * F18 * Lg, C)
         if self.arena is not None:
-            ops.groupnorm_scatter(x, W[f"{tt}.norm.w"], W[f"{tt}.norm.b"], self.arena.addrs(f"x18.{name}"), ws,
-                                  n_frames=nb * fl, hw=L, groups=self.cfg.norm_num_groups, eps=1e-6, fpb_in=fl,
-                                  fpb_out=F18, frame_off=nm + me * fl)
+            ops.groupnorm_scatter(x, W[f"{tt}.norm.w"], W[f"{tt}.norm.b"], self.arena.addrs(f"x18.{name}"),
+                                  self._gn_ws(), n_frames=nb * fl, hw=L, groups=self.cfg.norm_num_groups, eps=1e-6,
+                                  fpb_in=fl, fpb_out=F18, frame_off=nm + me * fl)
             with ops.timed_region(f"peer_barrier in C{C} L{L}"):
                 self.arena.barrier()
         else:
             gnl = self.buf("mm.gnl", nb * fl * L, C)
             self._gn(x, f"{tt}.norm", gnl, nb * fl, L, 1e-6, False)
-            g5 = gnl.view(nb, fl, R, Lg, C)
-            x5 = x18.view(nb, F18, Lg, C)
-            if sh.group_size > 1:
-                import torch.distributed as dist
-                send = self.buf("mm.a2a.s", R * nb * fl * Lg, C)
-                recv = self.buf("mm.a2a.r", R * nb * fl * Lg, C)
-                send.view(R, nb, fl, Lg, C).copy_(g5.permute(2, 0, 1, 3, 4))            # chunk d = my frames, pixel slice d
-                with ops.timed_region(f"a2a_frames_to_pixels C{C} L{L} R{R}"):
-                    dist.all_to_all_single(recv, send, group=sh.group)                 # chunk s = frames of rank s, my slice
-                x5[:, nm:].view(nb, R, fl, Lg, C).copy_(recv.view(R, nb, fl, Lg, C).permute(1, 0, 2, 3, 4))
-            else:                                                                      # emulation: peers = copies of me
-                x5[:, nm:].view(nb, R, fl, Lg, C).copy_(g5[:, :, me].unsqueeze(1).expand(nb, R, fl, Lg, C))
-        h = self.buf("mm.h", M18, C)
-        ops.gemm(x18, W[f"{tt}.proj_in.w"], h, bias=W[f"{tt}.proj_in.b"])
-        for a in range(2):
-            n = self._ln(h, f"{tb}.norms.{a}", "mm.ln", pe=W[f"{tb}.attention_blocks.{a}.pe"],
-                         pe_index=win["pe_index_all"], tokens_per_frame=Lg, frames=F18)
-            qkv = self.buf("mm.qkv", M18, 3 * C)
-            ops.gemm(n, W[f"{tb}.attention_blocks.{a}.qkv"], qkv)
-            o = self.buf("mm.attn", M18, C)
-            ops.temporal_attention(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], o, batch=nb, fq=F18, fk=F18, tokens=Lg,
-                                   heads=H)
-            h2 = self.buf(f"mm.h{a + 1}", M18, C)
-            ops.gemm(o, W[f"{tb}.attention_blocks.{a}.to_out.0.w"], h2,
-                     bias=W[f"{tb}.attention_blocks.{a}.to_out.0.b"], residual=h)
-            h = h2
-        h = self._ff(h, f"{tb}.ff", f"{tb}.ff_norm", "mm.h3")
+            # send chunk d = my frames, pixel slice d; received chunk s = frames of rank s, my pixel slice
+            got = self._exchange(gnl.view(nb, fl, R, Lg, C).permute(2, 0, 1, 3, 4),
+                                 f"a2a_frames_to_pixels C{C} L{L} R{R}")
+            x18.view(nb, F18, Lg, C)[:, nm:].view(nb, R, fl, Lg, C).copy_(got.permute(1, 0, 2, 3, 4))
+        h = self._motion_body(name, x18, Lg, F18, self.window["pe_index_all"])
         out = self.buf(out_tag, nb * fl * L, C)
         if self.arena is not None:
             recv = self.arena.local("recv", (nb * fl * L, C), self.dtype)
@@ -629,47 +599,59 @@ class DenoiseEngine:
             for b in range(nb):
                 ops.gemm(h[(b * F18 + nm) * Lg:(b + 1) * F18 * Lg], W[f"{tt}.proj_out.w"], y[b * f * Lg:(b + 1) * f * Lg],
                          bias=W[f"{tt}.proj_out.b"])
-            y5 = y.view(nb, R, fl, Lg, C)
-            if sh.group_size > 1:
-                import torch.distributed as dist
-                send = self.buf("mm.a2a.s", R * nb * fl * Lg, C)
-                recv = self.buf("mm.a2a.r", R * nb * fl * Lg, C)
-                send.view(R, nb, fl, Lg, C).copy_(y5.permute(1, 0, 2, 3, 4))            # chunk d = frames of rank d, my slice
-                with ops.timed_region(f"a2a_pixels_to_frames C{C} L{L} R{R}"):
-                    dist.all_to_all_single(recv, send, group=sh.group)                 # chunk s = my frames, pixel slice s
-                torch.add(recv.view(R, nb, fl, Lg, C).permute(1, 2, 0, 3, 4), x.view(nb, fl, R, Lg, C),
-                          out=out.view(nb, fl, R, Lg, C))
-            else:
-                mine = y5[:, me].unsqueeze(2).expand(nb, fl, R, Lg, C)                  # emulation: every slice = mine
-                torch.add(mine, x.view(nb, fl, R, Lg, C), out=out.view(nb, fl, R, Lg, C))
+            # send chunk d = frames of rank d, my pixel slice; received chunk s = my frames, pixel slice s
+            got = self._exchange(y.view(nb, R, fl, Lg, C).permute(1, 0, 2, 3, 4),
+                                 f"a2a_pixels_to_frames C{C} L{L} R{R}")
+            torch.add(got.permute(1, 2, 0, 3, 4), x.view(nb, fl, R, Lg, C), out=out.view(nb, fl, R, Lg, C))
         return out
 
-    def _motion(self, name: str, attn_name: str, x, level: int, C: int, out_tag: str):
-        if self.px:
-            return self._motion_px(name, x, level, C, out_tag)
-        W, win, H = self.W, self.window, self.cfg.heads
-        nb, nm, fl = self.nb, self.nm, self.fl
-        Fl = nm + fl
-        L = self.L(level)
-        Mm = nb * Fl * L
+    def _exchange(self, chunks: torch.Tensor, region: str) -> torch.Tensor:
+        """All-to-all of an exchange == "nccl" window: chunks[d] goes to rank d; returns chunks' shape with the chunk
+        received from rank s at [s].  An emulated group receives copies of the chunk this rank keeps."""
+        if self.shard.group_size == 1:
+            return chunks[self.me].unsqueeze(0).expand(chunks.shape)
+        import torch.distributed as dist
+        C = chunks.shape[-1]
+        send = self.buf("mm.a2a.s", chunks.numel() // C, C)
+        recv = self.buf("mm.a2a.r", chunks.numel() // C, C)
+        send.view(chunks.shape).copy_(chunks)
+        with ops.timed_region(region):
+            dist.all_to_all_single(recv, send, group=self.shard.group)
+        return recv.view(chunks.shape)
+
+    def _motion_body(self, name: str, x, tokens: int, frames: int, pe_index: torch.Tensor) -> torch.Tensor:
+        """proj_in, 2 x {LayerNorm + PE, QKV, temporal attention over the frames, to_out}, FF of a motion module on the
+        rows (cfg half, frame, pixel) of x, `frames` frames of `tokens` pixels each; returns the FF output."""
+        W, H = self.W, self.cfg.heads
+        M, C = x.shape
         tt = f"{name}.temporal_transformer"
         tb = f"{tt}.transformer_blocks.0"
-        gn18 = self.buf(f"{name}.gn18", Mm, C)          # frames [0, nm) were filled in begin_window
-        self._gn(x, f"{tt}.norm", gn18, nb * fl, L, 1e-6, False, fpb_in=fl, fpb_out=Fl, frame_off=nm)
-        h = self.buf("mm.h", Mm, C)
-        ops.gemm(gn18, W[f"{tt}.proj_in.w"], h, bias=W[f"{tt}.proj_in.b"])
+        h = self.buf("mm.h", M, C)
+        ops.gemm(x, W[f"{tt}.proj_in.w"], h, bias=W[f"{tt}.proj_in.b"])
         for a in range(2):
-            n = self._ln(h, f"{tb}.norms.{a}", "mm.ln", pe=W[f"{tb}.attention_blocks.{a}.pe"], pe_index=win["pe_index"],
-                         tokens_per_frame=L, frames=Fl)
-            qkv = self.buf("mm.qkv", Mm, 3 * C)
+            n = self._ln(h, f"{tb}.norms.{a}", "mm.ln", pe=W[f"{tb}.attention_blocks.{a}.pe"], pe_index=pe_index,
+                         tokens_per_frame=tokens, frames=frames)
+            qkv = self.buf("mm.qkv", M, 3 * C)
             ops.gemm(n, W[f"{tb}.attention_blocks.{a}.qkv"], qkv)
-            o = self.buf("mm.attn", Mm, C)
-            ops.temporal_attention(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], o, batch=nb, fq=Fl, fk=Fl, tokens=L, heads=H)
-            h2 = self.buf(f"mm.h{a + 1}", Mm, C)
+            o = self.buf("mm.attn", M, C)
+            ops.temporal_attention(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], o, batch=self.nb, fq=frames, fk=frames,
+                                   tokens=tokens, heads=H)
+            h2 = self.buf(f"mm.h{a + 1}", M, C)
             ops.gemm(o, W[f"{tb}.attention_blocks.{a}.to_out.0.w"], h2,
                      bias=W[f"{tb}.attention_blocks.{a}.to_out.0.b"], residual=h)
             h = h2
-        h = self._ff(h, f"{tb}.ff", f"{tb}.ff_norm", "mm.h3")
+        return self._ff(h, f"{tb}.ff", f"{tb}.ff_norm", "mm.h3")
+
+    def _motion(self, name: str, x, level: int, C: int, out_tag: str):
+        if self.px:
+            return self._motion_px(name, x, level, C, out_tag)
+        W, nb, nm, fl = self.W, self.nb, self.nm, self.fl
+        Fl = nm + fl
+        L = self.L(level)
+        tt = f"{name}.temporal_transformer"
+        gn18 = self.buf(f"{name}.gn18", nb * Fl * L, C)          # frames [0, nm) were filled in begin_window
+        self._gn(x, f"{tt}.norm", gn18, nb * fl, L, 1e-6, False, fpb_in=fl, fpb_out=Fl, frame_off=nm)
+        h = self._motion_body(name, gn18, L, Fl, self.window["pe_index"])
         out = self.buf(out_tag, nb * fl * L, C)
         for b in range(nb):                              # proj_out only on the real frames (drops motion frames)
             rows_in = slice((b * Fl + nm) * L, (b + 1) * Fl * L)
@@ -677,20 +659,23 @@ class DenoiseEngine:
             ops.gemm(h[rows_in], W[f"{tt}.proj_out.w"], out[rows_out], bias=W[f"{tt}.proj_out.b"], residual=x[rows_out])
         return out
 
-    def _cross_layer(self, b: BlockSpec, l: LayerSpec, x1, x2, level: int, out_tag: str):
+    def _cross_layer(self, b: BlockSpec, l: LayerSpec, x, level: int, out_tag: str):
+        """The layer's spatial transformer, then its audio and motion modules where it has them: the last module writes
+        out_tag, the others the shared lyr.* buffers."""
         C = b.channels
-        x = self._resnet(l.resnet, x1, x2, level, "lyr.rs")
-        x = self._spatial(l.attn, x, level, C, "lyr.sp")
-        x = self._audio(l.audio, x, level, C, l.audio_inner, b.depth, "lyr.au")
-        return self._motion(l.motion, l.attn, x, level, C, out_tag)
+        x = self._spatial(l.attn, x, level, C, "lyr.sp" if l.audio or l.motion_executed else out_tag)
+        if l.audio:
+            x = self._audio(l.audio, x, level, C, l.audio_inner, b.depth, "lyr.au" if l.motion_executed else out_tag)
+        if l.motion_executed:
+            x = self._motion(l.motion, x, level, C, out_tag)
+        return x
 
     # ------------------------------------------------------------------ forward
-    @torch.no_grad()
-    def _forward(self):
-        """One UNet3D forward over the local shard; reads self.latents, writes self.model_out [B*L0, 8]."""
+    def _walk(self):
+        """Time embedding -> conv_in -> down / mid / up blocks over the local rows; reads self.latents (or self.sample)
+        and the window, returns the last up block's features [B*L0, C0]."""
         W, cfg, B = self.W, self.cfg, self.B
-        h, w = self.h, self.w
-        L0 = h * w
+        L0 = self.h * self.w
         c0 = cfg.block_out_channels[0]
         # time embedding (unet_3d.py:565-588) -> SiLU(emb) -> all 22 time_emb_proj at once
         emb = self.buf("temb.sin", self.nb, c0)
@@ -701,61 +686,61 @@ class DenoiseEngine:
         ops.gemm(e1, W["time_embedding.linear_2.w"], e2, bias=W["time_embedding.linear_2.b"], silu=True)
         self.temb_all = self.buf("temb.all", self.nb, W.temb_total)
         ops.gemm(e2, W["temb_all.w"], self.temb_all, bias=W["temb_all.b"])
-        # conv_in + mask_cond_fea (unet_3d.py:603-605)
+        # conv_in (+ mask_cond_fea, unet_3d.py:603-605)
         cols = self.buf("im2col", B * L0, 64)
         ops.im2col_latent(self.sample if self.sample is not None else self.latents, cols, batch=self.nb)
         x = self.buf("x.conv_in", B * L0, c0)
-        ops.gemm(cols, W["conv_in.w"], x, bias=W["conv_in.b"], residual=self.window["mask_cond"])
-        skips: List[Tuple[torch.Tensor, int]] = [(x, c0)]
+        ops.gemm(cols, W["conv_in.w"], x, bias=W["conv_in.b"], residual=self.window.get("mask_cond"))
+        skips = [x]
         level = 0
         for b in W.blocks:
+            C = b.channels
             if b.kind in ("down_x", "down"):
                 for j, l in enumerate(b.layers):
                     tag = f"skip.{b.name}.{j}"
-                    if b.kind == "down_x":
-                        x = self._cross_layer(b, l, x, None, level, tag)
-                    else:
-                        x = self._resnet(l.resnet, x, None, level, tag)         # Q1b: motion module skipped
-                    skips.append((x, b.channels))
+                    x = self._resnet(l.resnet, x, None, level, "lyr.rs" if l.attn else tag)    # Q1b: resnet only
+                    if l.attn:
+                        x = self._cross_layer(b, l, x, level, tag)
+                    skips.append(x)
                 if b.downsampler:
                     hh, ww = self.level_hw[level]
-                    C = b.channels
                     planes = self.buf("ds.planes", B * hh * ww, C)
                     ops.phase_split(x.view(B, hh, ww, C), planes.view(4 * B, hh // 2, ww // 2, C))
                     level += 1
                     x = self.buf(f"skip.{b.name}.ds", B * self.L(level), C)
                     ops.conv3x3_stride2(planes.view(4 * B, hh // 2, ww // 2, C), W[f"{b.downsampler}.conv.w"], x,
                                         n=B, ho=hh // 2, wo=ww // 2, bias=W[f"{b.downsampler}.conv.b"])
-                    skips.append((x, C))
+                    skips.append(x)
             elif b.kind == "mid":
+                # UNetMidBlock3D/2DCrossAttn: resnets[0] -> the layer's transformer modules -> resnets[1]
                 x = self._resnet(b.extra_resnet, x, None, level, "mid.rs0")
-                l = b.layers[0]
-                C = b.channels
-                x = self._spatial(l.attn, x, level, C, "lyr.sp")
-                x = self._audio(l.audio, x, level, C, l.audio_inner, b.depth, "lyr.au")
-                x = self._motion(l.motion, l.attn, x, level, C, "mid.mm")
-                x = self._resnet(l.resnet, x, None, level, "mid.out")
+                x = self._cross_layer(b, b.layers[0], x, level, "mid.mm")
+                x = self._resnet(b.layers[0].resnet, x, None, level, "mid.out")
             else:
                 for j, l in enumerate(b.layers):
-                    sk, _ = skips.pop()
                     tag = f"up.{b.name}.{j % 2}"
-                    if b.kind == "up_x":
-                        x = self._cross_layer(b, l, x, sk, level, tag)
-                    else:
-                        x = self._resnet(l.resnet, x, sk, level, tag)           # Q1b
+                    x = self._resnet(l.resnet, x, skips.pop(), level, "lyr.rs" if l.attn else tag)    # Q1b
+                    if l.attn:
+                        x = self._cross_layer(b, l, x, level, tag)
                 if b.upsampler:
                     hh, ww = self.level_hw[level]
-                    C = b.channels
                     up = self.buf("us.up", B * 4 * hh * ww, C)
                     ops.upsample2x(x.view(B, hh, ww, C), up.view(B, 2 * hh, 2 * ww, C))
                     level -= 1
                     x = self.buf(f"up.{b.name}.us", B * self.L(level), C)
                     ops.conv3x3(up.view(B, 2 * hh, 2 * ww, C), W[f"{b.upsampler}.conv.w"], x,
                                 bias=W[f"{b.upsampler}.conv.b"])
-        t = self.buf("out.gn", B * L0, c0)
-        self._gn(x, "conv_norm_out", t, B, L0, cfg.norm_eps, True)
-        self.model_out = self.buf("out.conv", B * L0, 8)
-        ops.conv3x3(t.view(B, h, w, c0), W["conv_out.w"], self.model_out, bias=W["conv_out.b"])
+        return x
+
+    @torch.no_grad()
+    def _forward(self):
+        """One UNet3D forward over the local shard; reads self.latents, writes self.model_out [B*L0, 8]."""
+        x = self._walk()
+        B, h, w, c0 = self.B, self.h, self.w, self.cfg.block_out_channels[0]
+        t = self.buf("out.gn", B * h * w, c0)
+        self._gn(x, "conv_norm_out", t, B, h * w, self.cfg.norm_eps, True)
+        self.model_out = self.buf("out.conv", B * h * w, 8)
+        ops.conv3x3(t.view(B, h, w, c0), self.W["conv_out.w"], self.model_out, bias=self.W["conv_out.b"])
         return self.model_out
 
     @torch.no_grad()

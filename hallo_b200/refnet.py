@@ -4,27 +4,27 @@ unet_2d_blocks.py, transformer_2d.py:245-420, BasicTransformerBlock attention.py
 `norm1(hidden_states)` are the K/V banks of the denoising UNet's spatial attention (write mode,
 mutual_self_attention.py:223-232, 333-366).
 
-Same kernel plan as the denoising engine with the audio / motion modules and the reference-KV concat removed:
-  conv_in -> [resnet -> spatial transformer]* with skips -> mid -> up blocks; no conv_out (the reference returns the
-  last up block's features: post_process=False, :1344-1349).
+It is the denoising engine's kernel plan, `DenoiseEngine._walk`, over a block list without audio / motion modules
+(spec.build_blocks_2d) and a window without reference K/V; norm1 writes into the bank buffers.  There is no conv_out:
+the reference returns the last up block's features (post_process=False, :1344-1349).
 The six samples (2 CFG copies x (reference + nm motion frames)) ride the token layout as six "frames" of one batch.
 Reproduced quirk (Q10): the image tokens are tiled over the batch -- `encoder_hidden_states.repeat(tmp, 1, 1)`
 (mutual_self_attention.py:340-346) -- so sample n cross-attends to the tokens of CFG half n % 2, not n // 3.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Tuple
+from typing import List, Tuple
 
 import torch
 
 from . import ops
 from .engine import DenoiseEngine, PackedWeights, Shard
-from .spec import UNetConfig, reader_bank_order
+from .spec import build_blocks_2d, reader_bank_order
 
 
 class ReferenceNetWeights(PackedWeights):
     """Kernel-ready copies of the 682-entry UNet2D state dict (same packing as the 3D model's resnets / spatial blocks)."""
-    kind = "2d"
+    build_blocks = staticmethod(build_blocks_2d)
 
 
 class ReferenceNetEngine(DenoiseEngine):
@@ -33,113 +33,34 @@ class ReferenceNetEngine(DenoiseEngine):
         self.n = n_samples
         self.bank_names: List[Tuple[str, int]] = reader_bank_order(self.cfg)
 
-    def bank_buffer(self, name: str, L: int, C: int) -> torch.Tensor:
-        return self.buf(f"bank.{name}", self.n * L, C)
-
-    def _spatial2d(self, name: str, x, level: int, C: int, out_tag: str):
-        """Transformer2DModel + BasicTransformerBlock in write mode: norm1 output is banked, then plain self-attention,
-        image cross-attention (tiled tokens, Q10), GEGLU feed-forward."""
-        W, B, H = self.W, self.B, self.cfg.heads
-        L = self.L(level)
-        M = B * L
-        tb = f"{name}.transformer_blocks.0"
-        t = self.buf("tf.gn", M, C)
-        self._gn(x, f"{name}.norm", t, B, L, 1e-6, False)
-        h = self.buf("tf.h0", M, C)
-        ops.gemm(t, W[f"{name}.proj_in.w"], h, bias=W[f"{name}.proj_in.b"])
-        n1 = ops.layernorm(h, W[f"{tb}.norm1.w"], W[f"{tb}.norm1.b"], self.bank_buffer(name, L, C))   # the bank
-        qkv = self.buf("tf.qkv", M, 3 * C)
-        ops.gemm(n1, W[f"{tb}.attn1.qkv"], qkv)
-        a = self.buf("tf.attn", M, C)
-        ops.attention(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], a, heads=H, L=L)
-        h1 = self.buf("tf.h1", M, C)
-        ops.gemm(a, W[f"{tb}.attn1.to_out.0.w"], h1, bias=W[f"{tb}.attn1.to_out.0.b"], residual=h)
-        n2 = self._ln(h1, f"{tb}.norm2", "ln")
-        q2 = self.buf("tf.q2", M, C)
-        ops.gemm(n2, W[f"{tb}.attn2.q"], q2)
-        kvi = self.buf(f"{name}.kvimg", self.ehs_tiled.shape[0], 2 * C)
-        ops.gemm(self.ehs_tiled, W[f"{tb}.attn2.kv"], kvi)
-        a2 = self.buf("tf.attn", M, C)
-        ops.cross_attention(q2, kvi[:, :C], kvi[:, C:], a2, frames=B, tokens=L, heads=H, head_dim=C // H,
-                            n_keys=self.n_img_tokens, kv_frame_div=1)
-        h2 = self.buf("tf.h2", M, C)
-        ops.gemm(a2, W[f"{tb}.attn2.to_out.0.w"], h2, bias=W[f"{tb}.attn2.to_out.0.b"], residual=h1)
-        h3 = self._ff(h2, f"{tb}.ff", f"{tb}.norm3", "tf.h3")
-        out = self.buf(out_tag, M, C)
-        ops.gemm(h3, W[f"{name}.proj_out.w"], out, bias=W[f"{name}.proj_out.b"], residual=x)
-        return out
+    def _norm1_tag(self, name: str) -> str:
+        return f"bank.{name}"
 
     @torch.no_grad()
     def run(self, sample: torch.Tensor, timestep, encoder_hidden_states: torch.Tensor):
         """sample (n, 4, h, w), timestep scalar, encoder_hidden_states (n_ehs, tokens, 768) with n % n_ehs == 0.
         Returns (features of the last up block as fp32 (n, C0, h, w), {attn name: bank (n, L, C) in model dtype})."""
-        W, cfg, B = self.W, self.cfg, self.B
-        h, w = self.h, self.w
-        L0, c0 = h * w, cfg.block_out_channels[0]
+        W, win = self.W, self.window
         n = sample.shape[0]
         assert n == self.n and n % encoder_hidden_states.shape[0] == 0
         ehs = encoder_hidden_states.to(self.dev, self.dtype)
-        tiled = ehs.repeat(n // ehs.shape[0], 1, 1)                       # Q10: tiled over the batch, not interleaved
-        self.n_img_tokens = ehs.shape[1]
-        self.ehs_tiled = tiled.reshape(n * ehs.shape[1], ehs.shape[2]).contiguous()
+        tiled = ehs.repeat(n // ehs.shape[0], 1, 1).reshape(n * ehs.shape[1], ehs.shape[2])    # Q10: not interleaved
+        win["n_img_tokens"] = ehs.shape[1]
+        win["kvimg_frame_div"] = 1                                      # sample n reads image K/V rows of batch n
+        for b in W.blocks:
+            for l in b.layers:
+                if l.attn:
+                    kv = win[f"{l.attn}.kvimg"] = self.buf(f"{l.attn}.kvimg", tiled.shape[0], 2 * b.channels)
+                    ops.gemm(tiled, W[f"{l.attn}.transformer_blocks.0.attn2.kv"], kv)
         self.set_timestep(float(timestep) if not torch.is_tensor(timestep) else float(timestep.reshape(-1)[0]))
         self.step_idx.zero_()
         # the n samples become n frames of one batch entry: latents [1, Cl, n, h, w]
         self.latents.copy_(sample.to(self.dev, torch.float32).permute(1, 0, 2, 3).unsqueeze(0))
-        emb = self.buf("temb.sin", 1, c0)
-        ops.timestep_embed(self.t_table, self.step_idx, emb)
-        e1 = self.buf("temb.e1", 1, cfg.time_embed_dim)
-        ops.gemm(emb, W["time_embedding.linear_1.w"], e1, bias=W["time_embedding.linear_1.b"], silu=True)
-        e2 = self.buf("temb.e2", 1, cfg.time_embed_dim)
-        ops.gemm(e1, W["time_embedding.linear_2.w"], e2, bias=W["time_embedding.linear_2.b"], silu=True)
-        self.temb_all = self.buf("temb.all", 1, W.temb_total)
-        ops.gemm(e2, W["temb_all.w"], self.temb_all, bias=W["temb_all.b"])
-        cols = self.buf("im2col", B * L0, 64)
-        ops.im2col_latent(self.latents, cols, batch=1)
-        x = self.buf("x.conv_in", B * L0, c0)
-        ops.gemm(cols, W["conv_in.w"], x, bias=W["conv_in.b"])
-        skips = [x]
-        level = 0
-        for b in W.blocks:
-            C = b.channels
-            if b.kind in ("down_x", "down"):
-                for j, l in enumerate(b.layers):
-                    x = self._resnet(l.resnet, x, None, level, "lyr.rs" if l.attn else f"skip.{b.name}.{j}")
-                    if l.attn:
-                        x = self._spatial2d(l.attn, x, level, C, f"skip.{b.name}.{j}")
-                    skips.append(x)
-                if b.downsampler:
-                    hh, ww = self.level_hw[level]
-                    planes = self.buf("ds.planes", B * hh * ww, C)
-                    ops.phase_split(x.view(B, hh, ww, C), planes.view(4 * B, hh // 2, ww // 2, C))
-                    level += 1
-                    x = self.buf(f"skip.{b.name}.ds", B * self.L(level), C)
-                    ops.conv3x3_stride2(planes.view(4 * B, hh // 2, ww // 2, C), W[f"{b.downsampler}.conv.w"], x,
-                                        n=B, ho=hh // 2, wo=ww // 2, bias=W[f"{b.downsampler}.conv.b"])
-                    skips.append(x)
-            elif b.kind == "mid":
-                # UNetMidBlock2DCrossAttn: resnets[0] -> attentions[0] -> resnets[1]  (unet_2d_blocks.py:523-592)
-                x = self._resnet(b.extra_resnet, x, None, level, "mid.rs0")
-                x = self._spatial2d(b.layers[0].attn, x, level, C, "lyr.sp")
-                x = self._resnet(b.layers[0].resnet, x, None, level, "mid.out")
-            else:
-                for j, l in enumerate(b.layers):
-                    sk = skips.pop()
-                    x = self._resnet(l.resnet, x, sk, level, "lyr.rs" if l.attn else f"up.{b.name}.{j % 2}")
-                    if l.attn:
-                        x = self._spatial2d(l.attn, x, level, C, f"up.{b.name}.{j % 2}")
-                if b.upsampler:
-                    hh, ww = self.level_hw[level]
-                    up = self.buf("us.up", B * 4 * hh * ww, C)
-                    ops.upsample2x(x.view(B, hh, ww, C), up.view(B, 2 * hh, 2 * ww, C))
-                    level -= 1
-                    x = self.buf(f"up.{b.name}.us", B * self.L(level), C)
-                    ops.conv3x3(up.view(B, 2 * hh, 2 * ww, C), W[f"{b.upsampler}.conv.w"], x,
-                                bias=W[f"{b.upsampler}.conv.b"])
-        out = torch.empty(1, c0, n, h, w, device=self.dev, dtype=torch.float32)
+        x = self._walk()
+        out = torch.empty(1, self.cfg.block_out_channels[0], n, self.h, self.w, device=self.dev, dtype=torch.float32)
         ops.tokens_to_bcfhw(x, out)
-        banks: Dict[str, torch.Tensor] = {}
+        banks = {}
         for name, C in self.bank_names:
             L = self.L(self._block_level(name))
-            banks[name] = self.bank_buffer(name, L, C).view(n, L, C)
+            banks[name] = self.buf(self._norm1_tag(name), n * L, C).view(n, L, C)
         return out[0].permute(1, 0, 2, 3).contiguous(), banks

@@ -256,15 +256,21 @@ def param_spec(cfg: UNetConfig) -> List[Tuple[str, Tuple[int, ...], str]]:
     """[(state-dict key, shape, kind)] in the reference's registration order.  kind in
     {w, zero_w, b, norm_w, norm_b, pe}; zero_w marks tensors the reference zero-initialises
     (attention.py:691-701, motion_module.py:169-172)."""
+    keys = _stem_and_blocks(cfg, build_blocks(cfg))
+    c0 = cfg.block_out_channels[0]
+    _norm(keys, "conv_norm_out", c0)
+    _conv(keys, "conv_out", cfg.out_channels, c0, 3)
+    return keys
+
+
+def _stem_and_blocks(cfg: UNetConfig, blocks: List[BlockSpec]) -> List[Tuple[str, Tuple[int, ...], str]]:
     keys: List[Tuple[str, Tuple[int, ...], str]] = []
     temb = cfg.time_embed_dim
     c0 = cfg.block_out_channels[0]
     _conv(keys, "conv_in", c0, cfg.in_channels, 3)
     _lin(keys, "time_embedding.linear_1", temb, c0)
     _lin(keys, "time_embedding.linear_2", temb, temb)
-    blocks = build_blocks(cfg)
-
-    def emit_block(b: BlockSpec):
+    for b in blocks:
         # registration order in the reference: attentions, resnets, audio_modules, motion_modules, samplers
         # (key ORDER is irrelevant for strict loading; we keep a readable order).
         if b.extra_resnet is not None:
@@ -281,11 +287,6 @@ def param_spec(cfg: UNetConfig) -> List[Tuple[str, Tuple[int, ...], str]]:
             _conv(keys, f"{b.downsampler}.conv", b.channels, b.channels, 3)
         if b.upsampler:
             _conv(keys, f"{b.upsampler}.conv", b.channels, b.channels, 3)
-
-    for b in blocks:
-        emit_block(b)
-    _norm(keys, "conv_norm_out", c0)
-    _conv(keys, "conv_out", cfg.out_channels, c0, 3)
     return keys
 
 
@@ -319,26 +320,17 @@ def sinusoid_pe(max_len: int, d_model: int):
 # ---------------------------------------------------------------------------------------------
 # ReferenceNet (hallo/models/unet_2d_condition.py: the SD-1.5 UNet2D that produces the K/V banks)
 # ---------------------------------------------------------------------------------------------
+def build_blocks_2d(cfg: UNetConfig) -> List[BlockSpec]:
+    """The UNet2D's structural walk: the 3D walk with the audio and motion modules removed (same names)."""
+    blocks = build_blocks(cfg)
+    for b in blocks:
+        b.layers = [LayerSpec(l.resnet, attn=l.attn) for l in b.layers]
+    return blocks
+
+
 def param_spec_2d(cfg: UNetConfig) -> List[Tuple[str, Tuple[int, ...], str]]:
     """State-dict keys of the reference's UNet2DConditionModel built from the SD-1.5 config: the resnet / spatial
     transformer / sampler subset of the 3D walk (same names).  The reference deletes conv_norm_out / conv_act / conv_out
     (the ReferenceNet returns after the up blocks), so they are not part of the contract: 682 entries, verified against
     the instantiated reference class (tests/golden/unet2d_state_dict_keys.json)."""
-    keys: List[Tuple[str, Tuple[int, ...], str]] = []
-    temb = cfg.time_embed_dim
-    c0 = cfg.block_out_channels[0]
-    _conv(keys, "conv_in", c0, cfg.in_channels, 3)
-    _lin(keys, "time_embedding.linear_1", temb, c0)
-    _lin(keys, "time_embedding.linear_2", temb, temb)
-    for b in build_blocks(cfg):
-        if b.extra_resnet is not None:
-            _resnet(keys, b.extra_resnet, temb)
-        for l in b.layers:
-            _resnet(keys, l.resnet, temb)
-            if l.attn:
-                _spatial_tf(keys, l.attn, b.channels, cfg.cross_attention_dim)
-        if b.downsampler:
-            _conv(keys, f"{b.downsampler}.conv", b.channels, b.channels, 3)
-        if b.upsampler:
-            _conv(keys, f"{b.upsampler}.conv", b.channels, b.channels, 3)
-    return keys
+    return _stem_and_blocks(cfg, build_blocks_2d(cfg))
